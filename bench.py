@@ -334,7 +334,12 @@ def main():
                          "fused into the kernel (peer stores over NVLink) or by NCCL per GEMV")
     ap.add_argument("--sharded-extra", type=int, default=1, help="time BASELINE configs[4] sharded over the ranks")
     ap.add_argument("--detail", default=None, help="write a per-shape sweep (all formats, M=1..8, prefill) to this JSON file")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last step computed as DIR/<projection>.npy (float32, "
+                         "[layers, rows]; rank 0's outputs).  Inputs are seeded, so two builds can be compared output for output")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the GPU decode stack's outputs; --impl reference times a CPU sample and keeps none")
     args.warmup = max(args.warmup, 3)
     # stdout carries exactly one JSON line: native libraries that print there (NCCL's version banner) go to stderr
     sys.stdout.flush()
@@ -596,6 +601,14 @@ def main():
         got = outs[4][(rank if tp > 1 else 0) * F:][:F].cpu().numpy()[rows]  # outs[] stays indexed by matrix in every mode
         check = qo.max_norm_err(got, ref)
         assert check <= 1e-5, f"timed path disagrees with the oracle: {check}"
+        # before the extras below, which reuse the output buffers
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            layer_bytes = 4 * sum(outs[i].numel() for i in range(7))
+            dump_layers = min(args.layers, (64 << 20) // layer_bytes)   # the first layers, at most 64 MB in all
+            for j, (name, _, _) in enumerate(LLAMA7B):
+                c = torch.stack([outs[7 * l + j].reshape(-1) for l in range(dump_layers)])
+                np.save(os.path.join(args.dump_outputs, f"{name}.npy"), c.cpu().numpy().astype(np.float32))
 
     value = step_bytes * world * args.steps / (ms_dev * 1e-3) / 1e9
     e2e_value = step_bytes * world * args.steps / (ms_e2e * 1e-3) / 1e9

@@ -142,14 +142,26 @@ def test_new_entries_validate_before_any_cuda_call(lib):
     assert lib.qgemm_gemm_group_hinted(2, p, 1, wp, cp, fs, 1, 31, 1, 1, 0, None, p, 64) == BAD
 
 
-def test_no_cpu_fallback(lib):
-    """Without a B200 the compute entries must fail loudly, never compute on the host."""
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
+def check_no_cpu_fallback(lib):
     p = C.c_void_p(0x1000)
     assert lib.qgemm_gemm(2, p, p, p, 1, 1, 32, 1, 1, 0, None, 0, None) in (-3, -4)
     assert lib.qgemm_quantize_q8_1(p, p, 1, 32, 0, None) in (-3, -4)
+
+
+def test_no_cpu_fallback(lib):
+    """Without a B200 the compute entries must fail loudly, never compute on the host.  Where a GPU is present, the
+    check runs in a child process that is shown no device."""
+    import subprocess
+    import sys
+    import torch
+    if not torch.cuda.is_available():
+        check_no_cpu_fallback(lib)
+        return
+    path = os.pathsep.join([os.path.join(ROOT, "tests"), os.path.join(ROOT, "llama.cpp-quant-gemm_b200")])
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="", PYTHONPATH=path + os.pathsep + os.environ.get("PYTHONPATH", ""))
+    code = "import test_abi_host as t; from quant_gemm import _lib; t.check_no_cpu_fallback(_lib.lib())"
+    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=300)
+    assert out.returncode == 0, out.stdout[-2000:] + out.stderr[-2000:]
 
 
 def test_shard_range(lib):
