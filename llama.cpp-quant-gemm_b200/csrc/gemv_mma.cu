@@ -690,6 +690,17 @@ static cudaError_t launch_wide_wt(const GemvMmaWideParams& p, int nbw, int nt, s
     return launch_wide_inst<WT, 16, 2>(p, smem, grid, ms, st);
 }
 
+// Programmatic-dependent-launch mode of pass t0 of a multi-pass call.  QGEMM_INPUTS_READY (pdl = 2: compute at once, wait
+// only before exit) applies to the FIRST pass alone; the later passes of the same call wait for their predecessor before
+// they compute (pdl = 1: their weight stream still starts early).  With INPUTS_READY on every pass, three 8-token passes of
+// gemv_mma_kernel computed concurrently, and in about one call in three a few weight rows of the middle pass came out wrong
+// (q8_0, T = 24, K = 8192: all eight tokens of the affected rows, hundreds of times the rounding bound), while the same
+// passes run one after the other were exact.
+static int mma_pass_pdl(uint32_t flags, int t0) {
+    if (!(flags & QGEMM_WEIGHTS_STATIC)) return 0;
+    return (t0 == 0 && (flags & QGEMM_INPUTS_READY)) ? 2 : 1;
+}
+
 // T tokens in passes of 8 * NT
 cudaError_t launch_gemv_mma_wide(int wtype, const void* act, const void* wgt, float* C, int T, int F, int K, int64_t ldc_t,
                                  int64_t ldc_f, uint32_t flags, int num_sms, cudaStream_t st) {
@@ -712,7 +723,7 @@ cudaError_t launch_gemv_mma_wide(int wtype, const void* act, const void* wgt, fl
         p.C = C + (int64_t)t0 * ldc_t;
         p.T = tp; p.F = F; p.nb = nb; p.ldc_t = ldc_t; p.ldc_f = ldc_f;
         p.pitch = pitch; p.stages = stages;
-        p.pdl = (flags & QGEMM_WEIGHTS_STATIC) ? ((flags & QGEMM_INPUTS_READY) ? 2 : 1) : 0;
+        p.pdl = mma_pass_pdl(flags, t0);
         const size_t smem = fixed + (size_t)stages * kMmaRows * pitch;
         cudaError_t e;
         switch (wtype) {
@@ -754,7 +765,7 @@ cudaError_t launch_gemv_mma(int wtype, const void* act, const void* wgt, float* 
             p.C = C + (int64_t)t0 * ldc_t;
             p.T = min(8, T - t0); p.F = F; p.nb = nbk; p.ldc_t = ldc_t; p.ldc_f = ldc_f;
             p.pitch = bp; p.stages = stg;
-            p.pdl = (flags & QGEMM_WEIGHTS_STATIC) ? ((flags & QGEMM_INPUTS_READY) ? 2 : 1) : 0;
+            p.pdl = mma_pass_pdl(flags, t0);
             p.peer = peer ? *peer : PeerOut{};
             const bool ms = flags & QGEMM_MS_EXACT;
             cudaError_t e;
@@ -791,7 +802,7 @@ cudaError_t launch_gemv_mma(int wtype, const void* act, const void* wgt, float* 
         p.wgt = (const uint8_t*)wgt;
         p.C = C + (int64_t)t0 * ldc_t;
         p.T = min(8, T - t0); p.F = F; p.nb = nb; p.ldc_t = ldc_t; p.ldc_f = ldc_f;
-        p.pitch = pitch; p.stages = stages; p.span = span; p.pdl = (flags & QGEMM_WEIGHTS_STATIC) ? ((flags & QGEMM_INPUTS_READY) ? 2 : 1) : 0;
+        p.pitch = pitch; p.stages = stages; p.span = span; p.pdl = mma_pass_pdl(flags, t0);
         p.peer = peer ? *peer : PeerOut{};
         const bool ms = flags & QGEMM_MS_EXACT;
         cudaError_t e;
